@@ -34,6 +34,7 @@ VOCODER_FLOP_PER_CLIP = 0.0766e12                    # MelGAN generator
 VOCODER_BYTES_PER_CLIP = 0.73e9                      # algorithmic activation traffic of the MelGAN stack (fp32), SURVEY.md 8(d)
 DECODER_BYTES_PER_CLIP = 0.81e9                      # conv input + output activations in fp32, SURVEY.md 8(d)
 L_TOK, WAV_LEN = 265, 217088
+DUMP_LIMIT_BYTES = 64 << 20                          # --dump-outputs: at most this much in all
 
 
 def load_peaks():
@@ -299,6 +300,20 @@ def gpu_parity(dalle, voc, ref, K):
             "wav_rel_err": rel(wav, ref["wav"]), "tolerance": "token ids bit-exact; mel / wav 1e-3 relative (north_star)"}
 
 
+def dump_outputs(directory, out, limit=DUMP_LIMIT_BYTES):
+    """What pipeline.synthesize returned -- tokens (B,265), mel (B,1,80,848), wav (B,1,217088) -- as <directory>/<name>.npy in float32 (token
+    ids are exact).  Two builds run with the same arguments get the same inputs, so their dumps compare output for output.  A batch larger than
+    `limit` bytes is cut to a subset of clips drawn with a fixed seed, the same clips for every build, kept in batch order."""
+    import numpy as np
+    arrs = {k: v.detach().float().cpu() for k, v in out.items() if v is not None}
+    B = arrs["tokens"].shape[0]
+    keep = min(B, limit // sum(a[0].numel() * 4 for a in arrs.values()))
+    idx = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(directory, f"{k}.npy"), a[idx].numpy())
+
+
 def run_gpu_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -335,6 +350,7 @@ def run_gpu_arm(args):
         return out
 
     def timed(model, e2e: bool, steps: int):
+        """(ms, what the last step returned)"""
         torch.manual_seed(1234 + rank)
         if world > 1:
             dist.barrier()
@@ -343,7 +359,7 @@ def run_gpu_arm(args):
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record(st)
         for _ in range(steps):
-            one_clip_batch(model, e2e)
+            out = one_clip_batch(model, e2e)
         e.record(st)
         torch.cuda.synchronize()
         if world > 1:
@@ -351,7 +367,7 @@ def run_gpu_arm(args):
         ms = torch.tensor([s.elapsed_time(e)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     warm = max(args.warmup, 3)
     for _ in range(warm):
@@ -360,8 +376,10 @@ def run_gpu_arm(args):
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
-    ms_dev = timed(dalle, False, args.steps)
-    ms_e2e = timed(dalle, True, args.steps)
+    ms_dev, last = timed(dalle, False, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)  # before the next pass can reuse the engines' buffers
+    ms_e2e, _ = timed(dalle, True, args.steps)
     clk = clocks.stop() if rank == 0 else None
     clips = B * world * args.steps
     value, e2e_v = clips / (ms_dev * 1e-3), clips / (ms_e2e * 1e-3)
@@ -377,7 +395,7 @@ def run_gpu_arm(args):
         for _ in range(2):
             one_clip_batch(fast, False)
         n_fast = max(3, args.steps // 2)
-        ms_fast = timed(fast, False, n_fast)
+        ms_fast, _ = timed(fast, False, n_fast)
         f_ms = stage_times(fast, voc, cond_dev, B)
         modes = {"f16": {"value": B * world * n_fast / (ms_fast * 1e-3), "unit": "clips/s", "steps": n_fast, "sampler_only_clips_per_s": B / (f_ms[0] * 1e-3),
                          "note": "single-pass fp16 GEMM / attention operands (11-bit significand): logits ~1e-3 of fp32, ~99.6 % free-running token agreement "
@@ -563,7 +581,11 @@ def main():
     ap.add_argument("--no-modes", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--extras", default="train,configs2,configs4", help="which of the other BASELINE configs to measure in the same run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's tokens / mel / wav of the last timed step to DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -219,6 +219,121 @@ def gen_tokenizer_cases():
     print("tokenizer_cases:", [len(r) for r in raw])
 
 
+TOKENIZE_VARIANT_CAPTIONS = ["Two people talk while a dog barks and a car drives past on a wet road", "wind", "A B C d e f g h i j k l m n o p"]
+TOKENIZE_VARIANTS = [(77, True, 0), (256, False, -100), (12, True, 0)]  # (context_length, add_start_and_end, pad_value)
+CONFIG_CAPTIONS = ["a dog barks", "rain on a tin roof"]                  # what the caps.yaml test feeds prepare_condition
+
+
+def gen_tokenize_variants():
+    """clip.tokenize's option space (DALL-E style 256 without start/end tokens and -100 padding, a context short enough to truncate)."""
+    import json
+    import types
+    if "ftfy" not in sys.modules:
+        sys.modules["ftfy"] = types.SimpleNamespace(fix_text=lambda t: t)
+    rh.install_shims()
+    from sound_synthesis.modeling.modules.clip.simple_tokenizer import SimpleTokenizer
+    from sound_synthesis.modeling.modules.clip.clip import tokenize
+    cases = []
+    for ctx, sot_eot, pad in TOKENIZE_VARIANTS:
+        out = tokenize(TOKENIZE_VARIANT_CAPTIONS, context_length=ctx, add_start_and_end=sot_eot, with_mask=True, pad_value=pad, tokenizer=SimpleTokenizer(end_idx=49152))
+        cases.append({"context_length": ctx, "add_start_and_end": sot_eot, "pad_value": pad, "token": out["token"].tolist(), "mask": out["mask"].int().tolist()})
+    with open(os.path.join(GOLD, "tokenize_variants.json"), "w") as f:
+        json.dump({"captions": TOKENIZE_VARIANT_CAPTIONS, "cases": cases}, f)
+    print("tokenize_variants:", len(cases), "cases")
+
+
+def gen_bpe_merges():
+    """The merges of CLIP's BPE table that the reference's SimpleTokenizer applies while encoding every caption the CPU tests encode, with their
+    ranks.  Greedy lowest-rank-first merging never applies a pair outside this set, so a table holding these pairs at these ranks (and inert
+    pairs elsewhere, tests/helpers.py:golden_bpe_vocab) gives the full table's token ids for these captions."""
+    import json
+    import types
+    if "ftfy" not in sys.modules:
+        sys.modules["ftfy"] = types.SimpleNamespace(fix_text=lambda t: t)
+    rh.install_shims()
+    from sound_synthesis.modeling.modules.clip.simple_tokenizer import SimpleTokenizer
+
+    class Applied(dict):  # SimpleTokenizer.bpe asks `bigram not in self.bpe_ranks` of the pair it is about to merge
+        hits = set()
+
+        def __contains__(self, pair):
+            found = dict.__contains__(self, pair)
+            if found:
+                self.hits.add(pair)
+            return found
+    tk = SimpleTokenizer(end_idx=49152)
+    tk.bpe_ranks = Applied(tk.bpe_ranks)
+    captions = CAPTIONS + ["A dog barks"] + TOKENIZE_VARIANT_CAPTIONS + CONFIG_CAPTIONS
+    for c in captions:
+        tk.encode(c)
+    merges = sorted([tk.bpe_ranks[p], p[0], p[1]] for p in tk.bpe_ranks.hits)
+    with open(os.path.join(GOLD, "bpe_merges.json"), "w") as f:
+        json.dump({"n_merges": len(tk.bpe_ranks), "captions": captions, "merges": merges}, f, ensure_ascii=False)
+    print("bpe_merges:", len(merges), "of", len(tk.bpe_ranks))
+
+
+def gen_reference_configs():
+    """The `model` blocks of the reference's configs/caps.yaml and evaluation/caps_text.yaml."""
+    import json
+    with open(os.path.join(GOLD, "reference_configs.json"), "w") as f:
+        json.dump({name: rh.load_config(name)["model"] for name in ("configs/caps.yaml", "evaluation/caps_text.yaml")}, f, indent=1)
+    print("reference_configs: 2")
+
+
+def gen_host_policies():
+    """Host-side policies of the reference DiffusionTransformer: parameter / buffer names, the AdamW grouping of parameters(name='transformer'),
+    and sample_time('importance') before and after the switch-over (tests/test_cpu_host.py:test_host_policies_match_live_reference_module)."""
+    import json
+    K = 32
+    model, _ = rh.build_dalle(K=K, overrides=dict(n_layer=2, n_embd=128, n_head=2, condition_dim=64, dec_ch=32, dec_ch_mult=[1, 1, 1, 1, 2],
+                                                  dec_z_channels=64, embed_dim=64), seed=0)
+    ref = model.transformer
+    import ast
+    try:
+        ref.parameters(name="transformer")
+        groups_error = None
+    except AssertionError as e:  # "parameters {<names>} were not separated ...": store the names sorted (a set prints in hash order)
+        names, _, rest = str(e).partition(" were not")
+        groups_error = {"unseparated": sorted(ast.literal_eval(names[len("parameters "):])), "message": "were not" + rest}
+    sample_time = []
+    for count, hist in ((0.0, None), (11.0, torch.linspace(0.5, 9.0, 100))):
+        ref.Lt_count.fill_(count)
+        if hist is not None:
+            ref.Lt_history.copy_(hist)
+        torch.manual_seed(42)
+        t, pt = ref.sample_time(16, torch.device("cpu"), "importance")
+        sample_time.append({"t": t.tolist(), "pt": pt.tolist()})
+    with open(os.path.join(GOLD, "host_policies.json"), "w") as f:
+        json.dump({"state_dict_keys": sorted(ref.state_dict()), "named_groups_error": groups_error, "sample_time": sample_time}, f, indent=1)
+    print("host_policies:", len(ref.state_dict()), "keys")
+
+
+def gen_ema():
+    """The reference's EMA (engine/ema.py) over the update sequence of tests/test_cpu_host.py:test_device_resident_ema_matches_reference_ema
+    (same module, same seeds: keep the two in step)."""
+    rh.install_shims()
+    from sound_synthesis.engine.ema import EMA
+
+    class Net(torch.nn.Module):
+        def __init__(self):
+            super().__init__()
+            torch.manual_seed(0)
+            self.body = torch.nn.Sequential(torch.nn.Linear(16, 32), torch.nn.LayerNorm(32), torch.nn.Linear(32, 8))
+            self.register_buffer("steps", torch.zeros(3))
+
+        def get_ema_model(self):
+            return self.body
+    a = Net()
+    ema = EMA(a, decay=0.9, update_interval=2)
+    g = torch.Generator().manual_seed(1)
+    for it in range(7):
+        for p in a.parameters():
+            p.data.add_(torch.randn(p.shape, generator=g) * 0.01)
+        ema.update(it)
+    np.savez_compressed(os.path.join(GOLD, "ema_reference.npz"), **{k: v.numpy() for k, v in ema.state_dict().items()})
+    print("ema_reference:", len(ema.state_dict()), "tensors")
+
+
 def gen_clip_text():
     """N2: the reference's CLIPTextEmbedding.forward (Diffsound flags) on seeded weights.  CLIPTextEmbedding.__init__ downloads CLIP, so the instance
     is assembled by hand from the reference's own sub-modules (clip/model.py Transformer + LayerNorm) and driven through its unmodified forward()."""
@@ -294,6 +409,11 @@ if __name__ == "__main__":
     gen_decoder_tiny()
     gen_encoder_tiny()
     gen_tokenizer_cases()
+    gen_tokenize_variants()
+    gen_bpe_merges()
+    gen_reference_configs()
+    gen_host_policies()
+    gen_ema()
     gen_clip_text()
     gen_melgan()
     for f in sorted(os.listdir(GOLD)):

@@ -1,4 +1,6 @@
 """Shared helpers for the parity tests (CPU side)."""
+import gzip
+import json
 import os
 
 import numpy as np
@@ -13,6 +15,26 @@ def load_golden(name):
     sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
     rest = {k: z[k] for k in z.files if not k.startswith("sd.")}
     return sd, rest
+
+
+def load_golden_json(name):
+    with open(os.path.join(GOLD, name)) as f:
+        return json.load(f)
+
+
+def golden_bpe_vocab(directory):
+    """Write a BPE merge table of CLIP's length to `directory` and return its path.  It holds the merges that the reference tokenizer applies to
+    the golden captions (golden/bpe_merges.json) at their ranks in CLIP's table, and an inert pair at every other rank (U+2400 is outside the
+    byte alphabet, so no text forms it).  Lowest-rank-first merging only ever applies pairs of the stored set, so these captions get CLIP's token
+    ids, and the vocabulary keeps CLIP's size."""
+    g = load_golden_json("bpe_merges.json")
+    lines = [f"␀{r} ␀" for r in range(g["n_merges"])]
+    for r, a, b in g["merges"]:
+        lines[r] = f"{a} {b}"
+    path = os.path.join(str(directory), "bpe_golden.txt.gz")
+    with gzip.open(path, "wt", encoding="utf-8") as f:
+        f.write("\n".join(["#version: 0.2"] + lines) + "\n")
+    return path
 
 
 def portable_uniform(seed, shape):

@@ -116,8 +116,14 @@ def test_train_loss_and_gradients_match_reference():
     hist = torch.zeros(100).scatter_(0, torch.from_numpy(g["in_t"]), 0.1 * out["kl_loss"].detach() ** 2)
     assert torch.allclose(hist, torch.from_numpy(g["out_Lt_history"]), rtol=1e-5)
     out["loss"].backward()
+    gmax = max(float(abs(g["grad." + n]).max()) for n in names)
     for n in names:
         ref = torch.from_numpy(g["grad." + n])
+        if n.endswith("key.bias"):
+            # exactly zero (softmax is invariant to a shift common to all keys): both sides hold rounding noise (~1e-9) whose pattern depends
+            # on the host's CPU kernels and thread count, so check that it is noise rather than compare it element by element
+            assert max(float(leaf[n].grad.abs().max()), float(ref.abs().max())) < 1e-7 * gmax, n
+            continue
         err = (leaf[n].grad - ref).abs().max() / ref.abs().max().clamp_min(1e-12)
         assert err < 5e-4, (n, float(err))
 

@@ -67,7 +67,9 @@ def conv_out_pair(state, T, row0, col0, w, bias, scale, out=None):
 
 def gemm_desc(*, A, W, out, M, N, K, taps, lda, ldw, ldo, dtype=F16, batch=1, a_rows=0, a_cols=0, a_batch_stride=0, w_cols=0, out_batch_stride=0,
               bias=None, flags=0, alpha=1.0, split_off=0, dual_off=0, out_col_group=0, out_col_group_stride=0, A2=None, lda2=0, a2_rows=0, a2_cols=0,
-              a2_batch_stride=0, block_n=0, cta_pair=0, residual=None, ld_res=0, geo=None, amax_out=None, resident_w=0):
+              a2_batch_stride=0, block_n=0, cta_pair=0, residual=None, ld_res=0, geo=None, amax_out=None, resident_w=0, w_batch_stride=0,
+              res_batch_stride=0, max_ctas=0, a_mn=False, w_mn=False, use_tap_wcol=1):
+    assert use_tap_wcol and not (w_batch_stride or res_batch_stride or a_mn or w_mn), "batched W / residual, MN-major operands and default W columns are not emulated"
     assert not resident_w or (K == 64 and N <= 128 and len(taps) <= 32 and len(taps) * ((N + 15) // 16 * 16) * 128 <= 96 * 1024), "resident_w contract"
     assert dtype == F16
     a_rows, a_cols = a_rows or M, a_cols or K

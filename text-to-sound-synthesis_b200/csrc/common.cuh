@@ -5,24 +5,17 @@
 #include <cuda.h>
 #include <cstdint>
 #include <cstdio>
+#include "error.cuh"
 
 namespace dsb {
 
 // ---------------------------------------------------------------- error plumbing (host)
-void set_error(const char* fmt, ...);
 #define DSB_CHECK_CUDA(expr)                                                                    \
   do {                                                                                          \
     cudaError_t _e = (expr);                                                                    \
     if (_e != cudaSuccess) {                                                                    \
       dsb::set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(_e));     \
       return 1;                                                                                 \
-    }                                                                                           \
-  } while (0)
-#define DSB_REQUIRE(cond, ...)                                                                  \
-  do {                                                                                          \
-    if (!(cond)) {                                                                              \
-      dsb::set_error(__VA_ARGS__);                                                              \
-      return 2;                                                                                 \
     }                                                                                           \
   } while (0)
 

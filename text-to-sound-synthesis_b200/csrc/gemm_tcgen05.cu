@@ -9,18 +9,14 @@
 // * warp-specialised persistent kernel: warp0 = TMA producer, warp1 = tcgen05.mma issuer (+TMEM owner), warps2-5 = epilogue
 //   (TMEM -> registers -> bias / GELU2 / residual / tf32-round -> HBM); smem ring of kStages, 2 TMEM accumulator stages.
 #include "common.cuh"
-#include "diffsound_b200.h"
+#include "gemm_plan.cuh"
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
-#include <cstdlib>
 
 namespace dsb {
 
 constexpr int MN_BOX_BYTES_C = 64 * 128;
-constexpr int BLOCK_M = 128;
-constexpr int ROW_BYTES = 128;  // one swizzle-128B row of K per operand row
 constexpr int GEMM_THREADS = 320;  // warp0 TMA, warp1 MMA, warps 2..9 epilogue
-constexpr int MAX_TAPS = 32;
 constexpr int MN_BOX_BYTES = 64 * ROW_BYTES;  // one MN-major TMA box: 64 K rows x 64 two-byte columns
 constexpr int EPI_LD = 36;  // padded row stride (floats) of the epilogue transpose tile: 16-byte aligned rows, conflict-free
 
@@ -35,53 +31,6 @@ __device__ __forceinline__ uint64_t make_sw128_mnmajor_desc(uint32_t smem_addr) 
   d |= static_cast<uint64_t>(2) << 61;
   return d;
 }
-
-struct GemmParams {
-  int M, N, batch;
-  int tiles_m, tiles_n;
-  int kb_per_tap;  // ceil(Kc / BLOCK_K)
-  int block_k;     // elements per k-block (32 tf32 / 64 bf16)
-  int num_taps;
-  int tap_shift[MAX_TAPS];
-  int tap_acol[MAX_TAPS];
-  int tap_wcol[MAX_TAPS];  // W column offset per tap (default tap * Kc)
-  unsigned tap_a2_mask;    // bit i set: tap i reads the SECOND A tensor map (a fused GEMM over two activation buffers)
-  unsigned tap_share_mask; // resident-W kernel: bit i set: tap i multiplies the A box tap i-1 staged (same shift / column / operand)
-  int n_pad;               // resident-W kernel: rows of one W box = the MMA's N (N rounded up to 16)
-  int a_stages;            // resident-W kernel: depth of the A-box ring (whatever shared memory the resident weights leave, <= 12)
-  // fused split-fp16 pair kernel: f3_nsp spatial taps j, each with row shift tap_shift[j], hi-half columns tap_acol[j] (A) / tap_wcol[j] (W);
-  // the lo halves sit lo_a / lo_w columns further right
-  int f3_nsp, lo_a, lo_w;
-  long long split_off;     // DSB_GEMM_OUT_F16_SPLIT: offset of the lo half inside an output row
-  long long dual_off;      // DSB_GEMM_DUAL_LRELU: offset of the LeakyReLU(0.2) copy (hi at +dual_off, lo at +dual_off+split_off)
-  int ocg, ocg_stride;     // output column groups: logical column n lives at (n / ocg) * ocg_stride + n % ocg (0 = plain)
-  float* amax_out;         // optional: atomic max of |value stored| over the whole output (calibration of fp16 activation scales)
-  int kc;          // channels per tap
-  int b_batched;
-  const float* bias;
-  const float* residual;
-  long long ld_res, res_bstride;
-  void* out;
-  long long ldo, out_bstride;
-  int flags;
-  // optional row mask (padded conv geometry): row r -> p = r % geo_P; y = p / geo_Wp; x = p % geo_Wp;
-  // rows outside [y0,y1) x [x0,x1) are written as zeros.  geo_P == 0 disables.
-  int geo_P, geo_Wp, geo_y0, geo_y1, geo_x0, geo_x1;
-  float alpha;     // scale applied to the accumulator before bias (1.0 for Linear)
-  // MN-major operands (2-byte types, one tap): the operand lies in HBM as (K rows, MN columns) -- e.g. dY and X of a weight-gradient GEMM
-  // dW = dY^T X, which contract over the token dimension.  Loaded as 64-column x 64-row TMA boxes (SWIZZLE_128B), consumed through MN-major
-  // UMMA descriptors: no transposed copies.
-  int a_mn, b_mn;
-};
-
-template <int BLOCK_N>
-struct GemmSmem {
-  static constexpr int A_BYTES = BLOCK_M * ROW_BYTES;
-  static constexpr int B_BYTES = BLOCK_N * ROW_BYTES;
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = (BLOCK_N == 256) ? 4 : 6;
-  static constexpr int TOTAL = STAGES * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/ + 8 * 32 * 32 * 4 /*epilogue transpose tiles*/;
-};
 
 // One output tile's epilogue for one warp: TMEM -> registers -> XOR-swizzled smem transpose -> bias / activation / residual ->
 // coalesced global stores.  Shared by the 1-CTA and the CTA-pair kernels (row_base = first row of this warp's 32-row slab).
@@ -484,15 +433,6 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster_addr) {
   asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster_addr) : "memory");
 }
 
-struct PairSmem {
-  static constexpr int BLOCK_N = 256;
-  static constexpr int A_BYTES = BLOCK_M * ROW_BYTES;        // this CTA's 128 rows of A
-  static constexpr int B_BYTES = (BLOCK_N / 2) * ROW_BYTES;  // this CTA's half of the B tile
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = 6;
-  static constexpr int TOTAL = STAGES * STAGE_BYTES + 1024 + 256 + 8 * 32 * 32 * 4;
-};
-
 template <int KIND>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a2, const __grid_constant__ CUtensorMap tmap_b,
@@ -630,19 +570,7 @@ gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
 // product streams every operand tile once PER PASS (3 x (32 KB in + 32 KB out of shared memory per SM and 64-deep k-block): exactly the MMA time,
 // no slack).  Here one pipeline stage holds the four tiles of a k-block (A hi, A lo, W hi half, W lo half: 64 KB per CTA) and the issuer runs the
 // three passes off them: 64 KB in + 96 KB out per 1536 MMA cycles, so the shared-memory port is no longer co-critical and L2 traffic drops by a third.
-// BN = 256: 256 x 256 pair tiles (best MMA shape).  BN = 128: 256 x 128 pair tiles for problems with fewer 256-wide tiles than CTA pairs (the
-// N = 1024 projections at M = 4240: 68 tiles on 74 pairs) -- twice the tiles, so every pair runs two and the first tile's epilogue (a 128 KB residual
-// read-modify-write per CTA, several microseconds) hides under the second tile's mainloop instead of being fully exposed.
-template <int BN>
-struct PairSplitSmem {
-  static constexpr int BLOCK_N = BN;
-  static constexpr int TILE_A = BLOCK_M * ROW_BYTES;     // 16 KB: this CTA's 128 rows x 64 halves of A (hi or lo)
-  static constexpr int TILE_B = (BN / 2) * ROW_BYTES;    // this CTA's half of the W tile (hi or lo)
-  static constexpr int STAGE_BYTES = 2 * TILE_A + 2 * TILE_B;  // A hi | A lo | W hi | W lo
-  static constexpr int STAGES = BN == 256 ? 3 : 4;
-  static constexpr int TOTAL = STAGES * STAGE_BYTES + 1024 + 256 + 8 * 32 * 32 * 4;
-};
-
+// BN = 256: 256 x 256 pair tiles (best MMA shape).  BN = 128: 256 x 128 pair tiles for N <= 128 (the decoder's 128-channel convs).
 template <int BN>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 gemm_f16x3_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ GemmParams p) {
@@ -787,16 +715,6 @@ gemm_f16x3_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_
 // (num_taps x n_pad rows x 128 B, <= 96 KB) are loaded once per CTA and stay in shared memory, and consecutive taps that read the same A box
 // (the hi*hi / hi*lo passes of one spatial tap, or the folded [hi | lo] . [Wh | Wh], [hi | lo] . [Wl | 0] pair of a 32-channel row) share one
 // staged copy.  MMA N = n_pad (16..128), accumulators 2 x 128 TMEM columns, epilogue shared with the generic kernel.
-struct ResidentSmem {
-  static constexpr int A_BYTES = BLOCK_M * ROW_BYTES;
-  static constexpr int MAX_STAGES = 12;
-  static constexpr int W_MAX = 96 * 1024;
-  static constexpr int BAR_BYTES = 512;
-  static constexpr int EPI_BYTES = 8 * 32 * 32 * 4;
-  static constexpr int BUDGET = 227 * 1024 - 1024 /*static smem of the epilogue*/;
-  static constexpr int FIXED = 1024 /*align slack*/ + BAR_BYTES + EPI_BYTES;
-};
-
 template <int KIND>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 conv_resident_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a2, const __grid_constant__ CUtensorMap tmap_b,
@@ -985,44 +903,42 @@ int make_operand_map_mn(CUtensorMap* map, const void* ptr, int kind, long long m
   return 0;
 }
 
-template <int BLOCK_N, int KIND>
-static int launch(const CUtensorMap& ma, const CUtensorMap& ma2, const CUtensorMap& mb, const GemmParams& p, int max_ctas, cudaStream_t st) {
-  using S = GemmSmem<BLOCK_N>;
-  auto kern = gemm_tcgen05_kernel<BLOCK_N, KIND>;
+// One PDL launch of `Kern` with the plan's grid and shared memory; the first launch of each kernel raises its dynamic shared-memory limit
+// to `smem_limit`.
+template <auto Kern, typename... Maps>
+static int launch(const GemmPlan& g, int smem_limit, cudaStream_t st, const Maps&... maps) {
   static bool attr_done = false;
   if (!attr_done) {
-    DSB_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
+    DSB_CHECK_CUDA(cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_limit));
     attr_done = true;
   }
-  const int tiles = p.tiles_m * p.tiles_n * p.batch;
-  int grid = tiles < max_ctas ? tiles : max_ctas;
-  DSB_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(GEMM_THREADS), S::TOTAL, st, ma, ma2, mb, p));
+  DSB_CHECK_CUDA(launch_pdl(Kern, dim3(g.grid), dim3(GEMM_THREADS), g.smem_bytes, st, maps..., g.p));
   return 0;
 }
 
-template <int KIND>
-static int launch_pair(const CUtensorMap& ma, const CUtensorMap& ma2, const CUtensorMap& mb, const GemmParams& p, int max_ctas, cudaStream_t st) {
-  auto kern = gemm_tcgen05_pair_kernel<KIND>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    DSB_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, PairSmem::TOTAL));
-    attr_done = true;
+static int launch_plan(const GemmPlan& g, int kind, const CUtensorMap& ma, const CUtensorMap& ma2, const CUtensorMap& mb, cudaStream_t st) {
+  constexpr int TF32 = DSB_DTYPE_TF32, BF16 = DSB_DTYPE_BF16, F16 = DSB_DTYPE_F16;
+  switch (g.kernel) {
+    case CONV_RESIDENT:  // the A ring depth varies per launch: the limit covers every depth
+      return kind == BF16 ? launch<conv_resident_kernel<BF16>>(g, ResidentSmem::BUDGET, st, ma, ma2, mb)
+                          : launch<conv_resident_kernel<F16>>(g, ResidentSmem::BUDGET, st, ma, ma2, mb);
+    case GEMM_F16X3_PAIR:
+      return g.block_n == 128 ? launch<gemm_f16x3_pair_kernel<128>>(g, g.smem_bytes, st, ma, mb)
+                              : launch<gemm_f16x3_pair_kernel<256>>(g, g.smem_bytes, st, ma, mb);
+    case GEMM_PAIR:
+      if (kind == TF32) return launch<gemm_tcgen05_pair_kernel<TF32>>(g, g.smem_bytes, st, ma, ma2, mb);
+      if (kind == BF16) return launch<gemm_tcgen05_pair_kernel<BF16>>(g, g.smem_bytes, st, ma, ma2, mb);
+      return launch<gemm_tcgen05_pair_kernel<F16>>(g, g.smem_bytes, st, ma, ma2, mb);
+    default:  // GEMM_1CTA
+      if (g.block_n == 256) {
+        if (kind == TF32) return launch<gemm_tcgen05_kernel<256, TF32>>(g, g.smem_bytes, st, ma, ma2, mb);
+        if (kind == BF16) return launch<gemm_tcgen05_kernel<256, BF16>>(g, g.smem_bytes, st, ma, ma2, mb);
+        return launch<gemm_tcgen05_kernel<256, F16>>(g, g.smem_bytes, st, ma, ma2, mb);
+      }
+      if (kind == TF32) return launch<gemm_tcgen05_kernel<128, TF32>>(g, g.smem_bytes, st, ma, ma2, mb);
+      if (kind == BF16) return launch<gemm_tcgen05_kernel<128, BF16>>(g, g.smem_bytes, st, ma, ma2, mb);
+      return launch<gemm_tcgen05_kernel<128, F16>>(g, g.smem_bytes, st, ma, ma2, mb);
   }
-  const int tiles = p.tiles_m * p.tiles_n * p.batch;
-  int pairs = max_ctas / 2;
-  if (pairs < 1) pairs = 1;
-  if (tiles < pairs) pairs = tiles;
-  DSB_CHECK_CUDA(launch_pdl(kern, dim3(2 * pairs), dim3(GEMM_THREADS), PairSmem::TOTAL, st, ma, ma2, mb, p));
-  return 0;
-}
-
-static bool pair_default() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("DSB_GEMM_PAIR");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
 }
 
 }  // namespace dsb
@@ -1031,201 +947,23 @@ using namespace dsb;
 
 extern "C" int dsb_gemm_ex(const dsb_gemm_desc* d, void* stream) {
   DSB_REQUIRE(d != nullptr, "dsb_gemm_ex: null descriptor");
-  DSB_REQUIRE(d->M > 0 && d->N > 0 && d->K > 0 && d->batch > 0, "dsb_gemm_ex: bad shape M=%d N=%d K=%d batch=%d", d->M, d->N, d->K, d->batch);
-  DSB_REQUIRE(d->num_taps >= 1 && d->num_taps <= MAX_TAPS, "dsb_gemm_ex: num_taps=%d out of range", d->num_taps);
-  DSB_REQUIRE(d->dtype == DSB_DTYPE_TF32 || d->dtype == DSB_DTYPE_BF16 || d->dtype == DSB_DTYPE_F16,
-              "dsb_gemm_ex: dtype must be TF32, BF16 or F16 (use dsb_gemm_f32 for exact fp32)");
+  GemmPlan g;
+  if (const int rc = plan_gemm(*d, sm_count(), &g)) return rc;
+  const GemmParams& p = g.p;
   const int kind = d->dtype;
-  const int block_k = kind == DSB_DTYPE_TF32 ? 32 : 64;
-  GemmParams p{};
-  p.M = d->M; p.N = d->N; p.batch = d->batch;
-  p.tiles_m = (d->M + BLOCK_M - 1) / BLOCK_M;
-  p.kb_per_tap = (d->K + block_k - 1) / block_k;
-  p.block_k = block_k;
-  p.num_taps = d->num_taps;
-  for (int i = 0; i < MAX_TAPS; ++i) {
-    p.tap_shift[i] = i < d->num_taps ? d->tap_shift[i] : 0;
-    p.tap_acol[i] = i < d->num_taps ? d->tap_acol[i] : 0;
-    p.tap_wcol[i] = i < d->num_taps ? (d->use_tap_wcol ? d->tap_wcol[i] : i * d->K) : 0;
-  }
-  {
-    const int es_ = kind == DSB_DTYPE_TF32 ? 4 : 2;
-    for (int i = 0; i < d->num_taps; ++i)
-      DSB_REQUIRE((p.tap_acol[i] * es_) % 16 == 0 && (p.tap_wcol[i] * es_) % 16 == 0,
-                  "dsb_gemm_ex: tap %d starts at A column %d / W column %d: TMA box coordinates must be multiples of 16 bytes", i, p.tap_acol[i], p.tap_wcol[i]);
-  }
-  p.split_off = d->split_off > 0 ? d->split_off : d->N;
-  p.dual_off = d->dual_off;
-  p.amax_out = d->amax_out;
-  p.ocg = d->out_col_group; p.ocg_stride = d->out_col_group_stride;
-  p.tap_a2_mask = 0;
-  if (d->A2) {
-    for (int i = 0; i < d->num_taps; ++i)
-      if (d->tap_a2[i]) p.tap_a2_mask |= 1u << i;
-  }
-  DSB_REQUIRE(!(d->flags & DSB_GEMM_DUAL_LRELU) || ((d->flags & DSB_GEMM_OUT_F16_SPLIT) && d->dual_off > 0),
-              "dsb_gemm_ex: DSB_GEMM_DUAL_LRELU needs DSB_GEMM_OUT_F16_SPLIT and dual_off > 0");
-  DSB_REQUIRE(d->out_col_group == 0 || ((d->flags & DSB_GEMM_OUT_F16_SPLIT) && d->out_col_group % 4 == 0 && d->out_col_group_stride % 4 == 0 && !d->residual),
-              "dsb_gemm_ex: output column groups need the split-fp16 output, multiples of 4 and no residual");
-  p.kc = d->K;
-  p.b_batched = d->w_batch_stride != 0;
-  p.bias = d->bias; p.residual = d->residual; p.ld_res = d->ld_res; p.res_bstride = d->res_batch_stride;
-  p.out = d->out; p.ldo = d->ldo; p.out_bstride = d->out_batch_stride;
-  p.flags = d->flags;
-  p.geo_P = d->geo_P; p.geo_Wp = d->geo_Wp; p.geo_y0 = d->geo_y0; p.geo_y1 = d->geo_y1; p.geo_x0 = d->geo_x0; p.geo_x1 = d->geo_x1;
-  p.alpha = d->alpha == 0.0f ? 1.0f : d->alpha;
-  p.a_mn = d->a_mn_major != 0;
-  p.b_mn = d->b_mn_major != 0;
-  const bool any_mn = p.a_mn || p.b_mn;
-  DSB_REQUIRE(!any_mn || (kind != DSB_DTYPE_TF32 && d->num_taps == 1 && d->tap_shift[0] == 0 && d->tap_acol[0] == 0),
-              "dsb_gemm_ex: MN-major operands need a 2-byte dtype and a single unshifted tap");
-
-  const int sms = sm_count();
-  static const bool resident_ok = [] { const char* e = getenv("DSB_CONV_RESIDENT"); return !(e && e[0] == '0'); }();  // A/B switch
-  if (d->resident_w && resident_ok) {
-    DSB_REQUIRE(kind != DSB_DTYPE_TF32 && !any_mn && !p.b_batched && d->K == 64 && d->N <= 128 && d->use_tap_wcol,
-                "dsb_gemm_ex: resident_w needs a 2-byte dtype, K-major operands, K == 64 per tap, N <= 128, explicit tap_wcol and an unbatched W");
-    p.n_pad = (d->N + 15) / 16 * 16;
-    const int w_bytes = d->num_taps * p.n_pad * ROW_BYTES;
-    DSB_REQUIRE(w_bytes <= ResidentSmem::W_MAX, "dsb_gemm_ex: resident_w: %d taps x %d rows do not fit the %d KB weight area", d->num_taps, p.n_pad, ResidentSmem::W_MAX >> 10);
-    p.tap_share_mask = 0;
-    for (int i = 1; i < d->num_taps; ++i)
-      if (p.tap_shift[i] == p.tap_shift[i - 1] && p.tap_acol[i] == p.tap_acol[i - 1] && (((p.tap_a2_mask >> i) ^ (p.tap_a2_mask >> (i - 1))) & 1u) == 0)
-        p.tap_share_mask |= 1u << i;
-    p.tiles_n = 1;
-    CUtensorMap ma, mb;
-    static const int promo128 = [] { const char* e = getenv("DSB_CONV_RESIDENT_PROMO256"); return (e && e[0] == '1') ? 0 : 1; }();  // A/B switch
-    if (make_operand_map(&ma, d->A, kind, d->a_cols > 0 ? d->a_cols : d->K, d->a_rows > 0 ? d->a_rows : d->M, d->batch, d->lda, d->a_batch_stride, BLOCK_M, promo128)) return 3;
-    if (make_operand_map(&mb, d->W, kind, d->w_cols > 0 ? d->w_cols : (long long)d->K * d->num_taps, d->N, 1, d->ldw, 0, p.n_pad)) return 3;
-    CUtensorMap ma2 = ma;
-    if (p.tap_a2_mask &&
-        make_operand_map(&ma2, d->A2, kind, d->a2_cols > 0 ? d->a2_cols : d->K, d->a2_rows > 0 ? d->a2_rows : d->M, d->batch, d->lda2, d->a2_batch_stride, BLOCK_M, promo128))
-      return 3;
-    p.a_stages = (ResidentSmem::BUDGET - ResidentSmem::FIXED - w_bytes) / ResidentSmem::A_BYTES;
-    if (p.a_stages > ResidentSmem::MAX_STAGES) p.a_stages = ResidentSmem::MAX_STAGES;
-    {
-      static const int forced = [] { const char* e = getenv("DSB_CONV_RESIDENT_STAGES"); return e ? atoi(e) : 0; }();  // tuning runs
-      if (forced >= 2 && forced < p.a_stages) p.a_stages = forced;
-    }
-    const int smem_bytes = ResidentSmem::FIXED + w_bytes + p.a_stages * ResidentSmem::A_BYTES;
-    auto kern = kind == DSB_DTYPE_BF16 ? conv_resident_kernel<DSB_DTYPE_BF16> : conv_resident_kernel<DSB_DTYPE_F16>;
-    static bool attr_done[2] = {false, false};
-    if (!attr_done[kind == DSB_DTYPE_BF16]) {
-      DSB_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ResidentSmem::BUDGET));
-      attr_done[kind == DSB_DTYPE_BF16] = true;
-    }
-    const int tiles = p.tiles_m * p.batch;
-    const int cap = d->max_ctas > 0 ? d->max_ctas : sms;
-    DSB_CHECK_CUDA(launch_pdl(kern, dim3(tiles < cap ? tiles : cap), dim3(GEMM_THREADS), smem_bytes, reinterpret_cast<cudaStream_t>(stream), ma, ma2, mb, p));
-    return 0;
-  }
-  // tile-N choice: fewest waves, then the wider tile (less A re-read)
-  int block_n = d->block_n;
-  if (block_n == 0) {
-    static const int forced = [] { const char* e = getenv("DSB_GEMM_BLOCK_N"); return e ? atoi(e) : 0; }();  // A/B switch for tuning runs
-    if (forced == 128 || forced == 256) block_n = forced;
-  }
-  if (block_n == 0) {
-    if (d->N <= 128) block_n = 128;
-    else {
-      const long long t256 = (long long)p.tiles_m * ((d->N + 255) / 256) * d->batch;
-      const long long t128 = (long long)p.tiles_m * ((d->N + 127) / 128) * d->batch;
-      const long long cost256 = ((t256 + sms - 1) / sms) * 2, cost128 = ((t128 + sms - 1) / sms);
-      // where the 256-wide choice leads to the CTA-pair / fused split-fp16 kernels, 128-wide tiles only when they save at least a fifth of the
-      // waves: the pair tile has twice the arithmetic intensity per staged byte.  (A bare "fewer waves" rule picked the 1-CTA 128-wide kernel for 29 vs 30 waves
-      // at M = 67 840 and ran the N = 1024 / 4096 layers of a 256-clip batch at half the fused kernel's rate: tools/batch_scaling.py.)
-      const bool pair_possible = !any_mn && d->cta_pair >= 0 && d->M > BLOCK_M && (long long)d->K * d->num_taps >= 2048 && pair_default();
-      block_n = (pair_possible ? cost128 * 5 < cost256 * 4 : cost128 < cost256) ? 128 : 256;
-    }
-  }
-  DSB_REQUIRE(block_n == 128 || block_n == 256, "dsb_gemm_ex: block_n must be 0, 128 or 256");
-  // CTA pairs (cta_group::2, 256 x 256 tiles): default whenever the tile width is 256 and the problem is at least one pair tile tall
-  // measured (tools/gemm_microbench.py): pairs win once the mainloop dominates (K >= 2048: 33.3 -> 31.3 us at N=1024, K=4096) and
-  // lose ~1 us of extra prologue (cluster barriers) on short-K launches
-  DSB_REQUIRE(!(any_mn && d->cta_pair > 0), "dsb_gemm_ex: the cta_group::2 kernel takes K-major operands only");
-  const bool use_pair = !any_mn && (d->cta_pair > 0 || (d->cta_pair == 0 && d->block_n == 0 && block_n == 256 && d->M > BLOCK_M &&
-                                                        (long long)d->K * d->num_taps >= 2048 && pair_default()));
-  // split-fp16 tap list -- per spatial tap j the triple (shift_j, A lo, W hi), (shift_j, A hi, W lo), (shift_j, A hi, W hi) with constant hi -> lo column
-  // distances: run the three passes off ONE staged copy of the four tiles (Linear layers: one unshifted triple; convs: 9 / 3 / 2 shifted triples)
-  static const bool fuse_ok = [] { const char* e = getenv("DSB_GEMM_F16X3_FUSED"); return !(e && e[0] == '0'); }();
-  static const bool fuse_conv_ok = [] { const char* e = getenv("DSB_GEMM_F16X3_FUSED_CONV"); return !(e && e[0] == '0'); }();  // A/B switch
-  bool f3_pattern = fuse_ok && kind == DSB_DTYPE_F16 && d->num_taps % 3 == 0 && !p.tap_a2_mask && !p.b_batched && !any_mn && d->K % 64 == 0 && d->M > BLOCK_M;
-  int f3_lo_a = 0, f3_lo_w = 0;
-  if (f3_pattern) {
-    f3_lo_a = p.tap_acol[0] - p.tap_acol[1];
-    f3_lo_w = p.tap_wcol[1] - p.tap_wcol[0];
-    for (int j = 0; j < d->num_taps && f3_pattern; j += 3)
-      f3_pattern = p.tap_shift[j] == p.tap_shift[j + 1] && p.tap_shift[j] == p.tap_shift[j + 2] && p.tap_acol[j + 1] == p.tap_acol[j + 2] &&
-                   p.tap_acol[j] - p.tap_acol[j + 1] == f3_lo_a && p.tap_wcol[j] == p.tap_wcol[j + 2] && p.tap_wcol[j + 1] - p.tap_wcol[j] == f3_lo_w;
-    f3_pattern = f3_pattern && f3_lo_a > 0 && f3_lo_w > 0;
-  }
-  const bool f3_linear = f3_pattern && d->num_taps == 3 && p.tap_shift[0] == 0 && d->batch == 1;  // the denoiser's Linear layers (any N)
-  // conv form: whenever the caller left tile shape and pairing to the library
-  const bool f3_conv = f3_pattern && !f3_linear && fuse_conv_ok && d->block_n == 0 && d->cta_pair == 0;
-  const bool fused3 = f3_pattern && ((use_pair && f3_linear) || f3_conv);
-  bool fused_n128 = false;
-  const bool pair_tiles = use_pair || fused3;
-  if (pair_tiles) {
-    block_n = 256;
-    p.tiles_m = (d->M + 2 * BLOCK_M - 1) / (2 * BLOCK_M);
-    // fewer 256-wide tiles than CTA pairs: halve the tile width so that every pair runs two tiles and overlaps an epilogue with a mainloop
-    static const bool n128_ok = [] { const char* e = getenv("DSB_GEMM_F16X3_N128"); return e && e[0] == '1'; }();  // opt-in: measured SLOWER at B=16 (proj 25.2 -> 26.4 us, MLP2 76.4 -> 93.9 us): the narrower tile is shared-memory bound
-    if (fused3 && ((n128_ok && d->N >= 256 && (long long)p.tiles_m * ((d->N + 255) / 256) <= (d->max_ctas > 0 ? d->max_ctas : sms) / 2) || d->N <= 128)) {
-      fused_n128 = true;
-      block_n = 128;
-    }
-  }
-  p.tiles_n = (d->N + block_n - 1) / block_n;
-
   CUtensorMap ma, mb;
   const long long a_rows = d->a_rows > 0 ? d->a_rows : d->M;
   if (p.a_mn) {
     if (make_operand_map_mn(&ma, d->A, kind, a_rows, d->K, d->batch, d->lda, d->a_batch_stride)) return 3;
-  } else if (make_operand_map(&ma, d->A, kind, d->a_cols > 0 ? d->a_cols : d->K, a_rows, d->batch, d->lda, d->a_batch_stride, BLOCK_M)) return 3;
+  } else if (make_operand_map(&ma, d->A, kind, d->a_cols > 0 ? d->a_cols : d->K, a_rows, d->batch, d->lda, d->a_batch_stride, BLOCK_M, g.l2_promo_128)) return 3;
   if (p.b_mn) {
     if (make_operand_map_mn(&mb, d->W, kind, d->N, d->K, p.b_batched ? d->batch : 1, d->ldw, d->w_batch_stride)) return 3;
   } else if (make_operand_map(&mb, d->W, kind, d->w_cols > 0 ? d->w_cols : (long long)d->K * d->num_taps, d->N, p.b_batched ? d->batch : 1, d->ldw,
-                              d->w_batch_stride, pair_tiles ? block_n / 2 : block_n)) return 3;
+                              d->w_batch_stride, g.w_box_rows)) return 3;
   CUtensorMap ma2 = ma;
-  if (p.tap_a2_mask) {
-    DSB_REQUIRE(!any_mn, "dsb_gemm_ex: a second A operand is K-major only");
-    if (make_operand_map(&ma2, d->A2, kind, d->a2_cols > 0 ? d->a2_cols : d->K, d->a2_rows > 0 ? d->a2_rows : d->M, d->batch, d->lda2, d->a2_batch_stride, BLOCK_M)) return 3;
-  }
+  if (p.tap_a2_mask && make_operand_map(&ma2, d->A2, kind, d->a2_cols > 0 ? d->a2_cols : d->K, d->a2_rows > 0 ? d->a2_rows : d->M, d->batch, d->lda2,
+                                        d->a2_batch_stride, BLOCK_M, g.l2_promo_128))
+    return 3;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int max_ctas = d->max_ctas > 0 ? d->max_ctas : sms;
-  if (fused3) {
-    p.f3_nsp = d->num_taps / 3;
-    p.lo_a = f3_lo_a;
-    p.lo_w = f3_lo_w;
-    for (int j = 0; j < p.f3_nsp; ++j) {  // triple j -> spatial tap j: (row shift, hi-half column of A, hi-half column of W)
-      const int sh = p.tap_shift[3 * j], ac = p.tap_acol[3 * j + 1], wc = p.tap_wcol[3 * j];
-      p.tap_shift[j] = sh; p.tap_acol[j] = ac; p.tap_wcol[j] = wc;
-    }
-    const long long tiles = (long long)p.tiles_m * p.tiles_n * p.batch;
-    int pairs = max_ctas / 2;
-    if (pairs < 1) pairs = 1;
-    if (tiles < pairs) pairs = (int)tiles;
-    static bool attr_done[2] = {false, false};
-    if (fused_n128) {
-      if (!attr_done[0]) { DSB_CHECK_CUDA(cudaFuncSetAttribute(gemm_f16x3_pair_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, PairSplitSmem<128>::TOTAL)); attr_done[0] = true; }
-      DSB_CHECK_CUDA(launch_pdl(gemm_f16x3_pair_kernel<128>, dim3(2 * pairs), dim3(GEMM_THREADS), PairSplitSmem<128>::TOTAL, st, ma, mb, p));
-    } else {
-      if (!attr_done[1]) { DSB_CHECK_CUDA(cudaFuncSetAttribute(gemm_f16x3_pair_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, PairSplitSmem<256>::TOTAL)); attr_done[1] = true; }
-      DSB_CHECK_CUDA(launch_pdl(gemm_f16x3_pair_kernel<256>, dim3(2 * pairs), dim3(GEMM_THREADS), PairSplitSmem<256>::TOTAL, st, ma, mb, p));
-    }
-    return 0;
-  }
-  if (use_pair) {
-    if (kind == DSB_DTYPE_TF32) return launch_pair<DSB_DTYPE_TF32>(ma, ma2, mb, p, max_ctas, st);
-    if (kind == DSB_DTYPE_BF16) return launch_pair<DSB_DTYPE_BF16>(ma, ma2, mb, p, max_ctas, st);
-    return launch_pair<DSB_DTYPE_F16>(ma, ma2, mb, p, max_ctas, st);
-  }
-  if (block_n == 256) {
-    if (kind == DSB_DTYPE_TF32) return launch<256, DSB_DTYPE_TF32>(ma, ma2, mb, p, max_ctas, st);
-    if (kind == DSB_DTYPE_BF16) return launch<256, DSB_DTYPE_BF16>(ma, ma2, mb, p, max_ctas, st);
-    return launch<256, DSB_DTYPE_F16>(ma, ma2, mb, p, max_ctas, st);
-  }
-  if (kind == DSB_DTYPE_TF32) return launch<128, DSB_DTYPE_TF32>(ma, ma2, mb, p, max_ctas, st);
-  if (kind == DSB_DTYPE_BF16) return launch<128, DSB_DTYPE_BF16>(ma, ma2, mb, p, max_ctas, st);
-  return launch<128, DSB_DTYPE_F16>(ma, ma2, mb, p, max_ctas, st);
+  return launch_plan(g, kind, ma, ma2, mb, st);
 }

@@ -168,58 +168,40 @@ def gemm(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None, 
     out_bf16 = out.dtype == torch.bfloat16
     if split_out and (out.dtype != torch.float16 or batched):
         raise RuntimeError("gemm: split_out writes an fp16 (hi | lo) pair and is not batched")
-    d = _lib.GemmDesc()
-    d.A, d.W, d.bias, d.residual, d.out = a.data_ptr(), w.data_ptr(), _ptr(bias), _ptr(residual), out.data_ptr()
-    d.M, d.N, d.K, d.batch = M, N, K, batch
-    d.a_rows = a_rows
-    d.lda, d.ldw, d.ldo = a.stride(-2), w.stride(-2), out.stride(-2)
-    d.ld_res = residual.stride(-2) if residual is not None else 0
-    d.a_batch_stride = a.stride(0) if batched else 0
-    d.w_batch_stride = w.stride(0) if w.dim() == 3 else 0
-    d.out_batch_stride = out.stride(0) if batched else 0
-    d.res_batch_stride = residual.stride(0) if (residual is not None and batched) else 0
-    d.dtype = dtype
-    d.flags = (GELU2 if gelu else 0) | (ROUND_TF32 if round_out else 0) | (OUT_BF16 if out_bf16 else 0) | (LRELU if lrelu else 0) | (TANH if tanh else 0) | (RES_BEFORE_ACT if res_before_act else 0) | (OUT_F16 if out_f16 else 0) | (OUT_F16_SPLIT if split_out else 0)
-    if split_out:
-        d.split_off = N
-    if tap_wcol is not None:
-        d.use_tap_wcol = 1
-        d.w_cols = w.shape[-1]
-        for i, c_ in enumerate(tap_wcol):
-            d.tap_wcol[i] = int(c_)
-    d.num_taps = ntaps
-    for i, s in enumerate(taps or [0]):
-        d.tap_shift[i] = int(s)
-        d.tap_acol[i] = int(tap_acol[i]) if tap_acol is not None else 0
-    d.a_cols = a_cols
-    if geo is not None:
-        d.geo_P, d.geo_Wp, d.geo_y0, d.geo_y1, d.geo_x0, d.geo_x1 = [int(v) for v in geo]
-    d.alpha = alpha
-    d.block_n, d.max_ctas, d.cta_pair = block_n, max_ctas, cta_pair
-    d.a_mn_major, d.b_mn_major = int(a_mn), int(w_mn)
-    _lib.check(_lib.lib().dsb_gemm_ex(C.byref(d), _stream()), "dsb_gemm_ex")
+    flags = (GELU2 if gelu else 0) | (ROUND_TF32 if round_out else 0) | (OUT_BF16 if out_bf16 else 0) | (LRELU if lrelu else 0) | (TANH if tanh else 0) | (RES_BEFORE_ACT if res_before_act else 0) | (OUT_F16 if out_f16 else 0) | (OUT_F16_SPLIT if split_out else 0)
+    tap_list = [(s, tap_acol[i] if tap_acol is not None else 0, tap_wcol[i] if tap_wcol is not None else 0, 0) for i, s in enumerate(taps or [0])]
+    gemm_desc(A=a.data_ptr(), W=w.data_ptr(), out=out.data_ptr(), M=M, N=N, K=K, batch=batch, dtype=dtype, flags=flags, alpha=alpha, taps=tap_list,
+              use_tap_wcol=int(tap_wcol is not None), w_cols=w.shape[-1] if tap_wcol is not None else 0,
+              a_rows=a_rows, a_cols=a_cols, lda=a.stride(-2), ldw=w.stride(-2), ldo=out.stride(-2),
+              a_batch_stride=a.stride(0) if batched else 0, w_batch_stride=w.stride(0) if w.dim() == 3 else 0, out_batch_stride=out.stride(0) if batched else 0,
+              bias=bias, residual=_ptr(residual), ld_res=residual.stride(-2) if residual is not None else 0,
+              res_batch_stride=residual.stride(0) if (residual is not None and batched) else 0, split_off=N if split_out else 0, geo=geo,
+              block_n=block_n, max_ctas=max_ctas, cta_pair=cta_pair, a_mn=a_mn, w_mn=w_mn)
     return out
 
 
 def gemm_desc(*, A, W, out, M, N, K, taps, lda, ldw, ldo, dtype=F16, batch=1, a_rows=0, a_cols=0, a_batch_stride=0, w_cols=0, out_batch_stride=0,
               bias=None, flags=0, alpha=1.0, split_off=0, dual_off=0, out_col_group=0, out_col_group_stride=0, A2=None, lda2=0, a2_rows=0, a2_cols=0,
-              a2_batch_stride=0, block_n=0, cta_pair=0, residual=None, ld_res=0, geo=None, amax_out=None, resident_w=0):
-    """Thin front end of dsb_gemm_ex for callers that lay out their own buffers (the MelGAN / SpecVQGAN state buffers): A / W / out / A2 are
-    raw device addresses (ints: tensor.data_ptr() plus a byte offset), sizes and strides in elements; taps = [(row_shift, a_col, w_col, use_a2), ...]."""
+              a2_batch_stride=0, block_n=0, cta_pair=0, residual=None, ld_res=0, geo=None, amax_out=None, resident_w=0, w_batch_stride=0,
+              res_batch_stride=0, max_ctas=0, a_mn=False, w_mn=False, use_tap_wcol=1):
+    """Descriptor front end of dsb_gemm_ex, for callers that lay out their own buffers (the MelGAN / SpecVQGAN state buffers) and for gemm(): A / W /
+    out / A2 / residual are raw device addresses (ints: tensor.data_ptr() plus a byte offset), sizes and strides in elements;
+    taps = [(row_shift, a_col, w_col, use_a2), ...]; use_tap_wcol=0 ignores w_col and reads W columns [i*K, (i+1)*K) for tap i."""
     d = _lib.GemmDesc()
     d.A, d.W, d.out, d.bias, d.A2 = A, W, out, _ptr(bias), A2
     d.M, d.N, d.K, d.batch = M, N, K, batch
     d.a_rows, d.a_cols, d.lda, d.ldw, d.ldo = a_rows, a_cols, lda, ldw, ldo
-    d.a_batch_stride, d.out_batch_stride = a_batch_stride, out_batch_stride
+    d.a_batch_stride, d.w_batch_stride, d.out_batch_stride = a_batch_stride, w_batch_stride, out_batch_stride
     d.dtype, d.flags, d.alpha = dtype, flags, alpha
     d.num_taps = len(taps)
-    d.use_tap_wcol, d.w_cols = 1, w_cols
+    d.use_tap_wcol, d.w_cols = use_tap_wcol, w_cols
     for i, (sh, ac, wc, a2) in enumerate(taps):
         d.tap_shift[i], d.tap_acol[i], d.tap_wcol[i], d.tap_a2[i] = int(sh), int(ac), int(wc), int(a2)
     d.split_off, d.dual_off, d.out_col_group, d.out_col_group_stride = split_off, dual_off, out_col_group, out_col_group_stride
     d.lda2, d.a2_rows, d.a2_cols, d.a2_batch_stride = lda2, a2_rows, a2_cols, a2_batch_stride
-    d.block_n, d.cta_pair = block_n, cta_pair
-    d.residual, d.ld_res = residual, ld_res
+    d.block_n, d.max_ctas, d.cta_pair = block_n, max_ctas, cta_pair
+    d.a_mn_major, d.b_mn_major = int(a_mn), int(w_mn)
+    d.residual, d.ld_res, d.res_batch_stride = residual, ld_res, res_batch_stride
     d.amax_out = _ptr(amax_out)
     d.resident_w = int(resident_w)
     if geo is not None:
